@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this engine (one rank per GPU under torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on the host cores
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's waveform(s) as DIR/<name>.npy
 
 A step = one `TextToSpeech.tts_with_preset(preset='standard')` call (256 AR candidates, 200 diffusion iterations,
 k=1) on the 53-word paragraph of SURVEY §8d config 3 (T=169 BPE tokens, N=430 mel tokens => S=1872 mel frames,
@@ -197,6 +198,25 @@ def config5_tokens(base):
     return [[base[i % len(base)] for i in range(n)] for n in (169, 193, 217, 241, 265, 289, 313, 337)]
 
 
+DUMP_BYTES = 63 << 20          # --dump-outputs: at most 64 MB on disk, .npy headers included
+
+
+def dump_outputs(d, wav):
+    """Writes what the timed call returned (the waveform, or one per candidate for k > 1) as float32 DIR/<name>.npy, so
+    that two builds can be compared output for output. Beyond DUMP_BYTES in all, every array is cut to the same fixed,
+    seeded share of its elements."""
+    import numpy as np
+    wavs = wav if isinstance(wav, list) else [wav]
+    arrays = {"wav" if len(wavs) == 1 else "wav_%d" % i: w.float().numpy() for i, w in enumerate(wavs)}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = np.random.default_rng(0).permutation(a.size)[:a.size * DUMP_BYTES // total]
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 ITERS = {"standard": 200, "fast": 80, "ultra_fast": 30, "high_quality": 400}
 NCAND = {"standard": 256, "high_quality": 256, "fast": 96, "ultra_fast": 16}
 
@@ -287,6 +307,8 @@ def run_engine(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wav)
     B = NCAND[preset]
     iters = ITERS[preset]
     h2d = sum(t.numel() * 4 for t in cl_host) * len(utt) + sum(4 * (len(u) + 1) for u in utt)
@@ -450,7 +472,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
     ap.add_argument("--cpu-timeout", type=int, default=240, help="seconds allowed per baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the waveform(s) of the last timed step as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,8 +1,8 @@
 """CPU: the tokenizer's text cleaners (tortoise_tts_b200/cleaners.py) against the known-answer table of the upstream
 cleaners the reference vendors (tortoise/utils/tokenizer.py:11-157 is keithito/tacotron `text/cleaners.py` + `numbers.py`;
 the expectations below are that project's published unit-test vectors for normalize_numbers, which the reference does
-not ship) and, where the reference tree is importable, against the reference's own `english_cleaners` on number-free
-text (`inflect` is absent from this image, so the reference cannot expand numbers here)."""
+not ship) and against the reference's own `english_cleaners` on number-free text (`inflect` is absent from this image,
+so the reference cannot expand numbers here)."""
 import pytest
 
 from tortoise_tts_b200 import cleaners as c
@@ -40,16 +40,20 @@ def test_english_cleaners_chain():
     assert c.to_ascii("plain ascii 123") == "plain ascii 123"
 
 
-@pytest.mark.reference
 def test_against_reference_cleaners_without_numbers():
-    from oracle import ref_shims
-    ref_shims.load_reference()
-    from tortoise.utils import tokenizer as rt
+    """Digests of the reference's english_cleaners / basic_cleaners outputs are stored (tests/ref_golden.py)."""
     import random
+    import ref_golden as rg
     rng = random.Random(0)
     words = ["Mr.", "Mrs.", "Dr.", "St.", "the", "Quick", "BROWN", "fox,", '"quoted"', "co.", "Ltd.", "hello\tworld",
              "Gen.", "lt.", "end.", "  spaced  ", "semi;colon", "Capt.", "jr.", "x"]
-    for _ in range(200):
+
+    def reference(s):
+        from oracle import ref_shims
+        ref_shims.load_reference()
+        from tortoise.utils import tokenizer as rt
+        return [rt.english_cleaners(s), rt.basic_cleaners(s)]
+    for i in range(200):
         s = " ".join(rng.choice(words) for _ in range(rng.randint(1, 12)))
-        assert c.english_cleaners(s) == rt.english_cleaners(s), s
-        assert c.basic_cleaners(s) == rt.basic_cleaners(s), s
+        assert rg.hexdigest([c.english_cleaners(s), c.basic_cleaners(s)]) == \
+            rg.digest("cleaners_%d" % i, lambda: reference(s)), s

@@ -1,11 +1,9 @@
-"""Long-form text splitter (tortoise_tts_b200/text.py) against the reference's own known-answer tests, committed
-reference outputs on seeded synthetic texts, and (where /root/reference exists) the reference function itself."""
+"""Long-form text splitter (tortoise_tts_b200/text.py) against the reference's own known-answer tests and committed
+outputs of the reference function on seeded synthetic texts."""
 import importlib.util
 import json
 import os
 import random
-
-import pytest
 
 from tortoise_tts_b200.text import split_and_recombine_text, utterance_plan
 
@@ -65,23 +63,30 @@ def test_utterance_plan():
     assert utterance_plan(3, 8) == [0, 1, 2]
 
 
-@pytest.mark.reference
 def test_against_reference_function():
-    path = "/root/reference/tortoise/utils/text.py"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    spec = importlib.util.spec_from_file_location("ref_text", path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    """Digests of the reference function's chunks on seeded random texts and on its own sample story are stored
+    (tests/ref_golden.py); the story itself is stored with them."""
+    import ref_golden as rg
+
+    def reference_module():
+        from oracle.ref_shims import REFERENCE_ROOT
+        spec = importlib.util.spec_from_file_location("ref_text", os.path.join(REFERENCE_ROOT, "tortoise", "utils", "text.py"))
+        ref = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(ref)
+        return ref
     rng = random.Random(99)
     alphabet = 'abc de. fg! "hi?" \n\n jk... “lm” ,;:x' + "y" * 5
-    for _ in range(400):
+    for i in range(400):
         text = "".join(rng.choice(alphabet) for _ in range(rng.randint(0, 500)))
         d = rng.choice([5, 20, 60, 200])
         m = d + rng.choice([1, 10, 100])
-        assert split_and_recombine_text(text, d, m) == ref.split_and_recombine_text(text, d, m), repr(text)
-    story = os.path.join(os.path.dirname(path), "..", "data", "riding_hood.txt")
-    if os.path.exists(story):
-        with open(story) as f:
-            t = f.read()
-        assert split_and_recombine_text(t) == ref.split_and_recombine_text(t)
+        want = rg.digest("text_split_%d" % i, lambda: reference_module().split_and_recombine_text(text, d, m))
+        assert rg.hexdigest(split_and_recombine_text(text, d, m)) == want, repr(text)
+
+    def reference_story():
+        from oracle.ref_shims import REFERENCE_ROOT
+        with open(os.path.join(REFERENCE_ROOT, "tortoise", "data", "riding_hood.txt")) as f:
+            return f.read()
+    t = rg.value("text_split_story", reference_story)
+    want = rg.digest("text_split_story_chunks", lambda: reference_module().split_and_recombine_text(t))
+    assert rg.hexdigest(split_and_recombine_text(t)) == want
